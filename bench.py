@@ -18,7 +18,9 @@ import subprocess
 import sys
 import threading
 import time
+import zlib
 
+import numpy as np
 import torch
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
@@ -42,14 +44,29 @@ WORKLOADS = {
 }
 
 
+DUMP_MAX_ELEMENTS = 5_000_000      # per output: a run dumps at most three (latents, decoded frames, encoded latents) = 60 MB
+
+
+def dump_sample(t, name):
+    """`t` as float32 on the host for --dump-outputs: whole up to DUMP_MAX_ELEMENTS, else that many elements (flattened) at positions
+    drawn from a generator seeded by `name`, so that every run with the same arguments samples the same positions."""
+    flat = t.detach().reshape(-1)
+    if flat.numel() > DUMP_MAX_ELEMENTS:
+        g = torch.Generator().manual_seed(zlib.crc32(name.encode()))
+        idx = torch.randint(0, flat.numel(), (DUMP_MAX_ELEMENTS,), generator=g).sort().values
+        return flat[idx.to(flat.device)].float().cpu()
+    return t.detach().float().cpu()
+
+
 def hy_flops_forward(cfg, L, Lt):
     D, nl, ns = cfg["hidden_size"], cfg["mm_double_blocks_depth"], cfg.get("mm_single_blocks_depth", 0)
     n = L + Lt
     return (nl + ns) * (4.0 * n * n * D + 8.0 * n * D * D + 16.0 * n * D * D)
 
 
-def measure_hunyuan(workload, steps, warmup, rank, world, local_rank, dev, dist, with_vae=True, cfg_split=False):
-    """Hunyuan Video denoise-step measurement (same JSON contract, steps of cond+uncond forwards + CFG + Euler) -> result dict."""
+def measure_hunyuan(workload, steps, warmup, rank, world, local_rank, dev, dist, with_vae=True, cfg_split=False, outputs=None):
+    """Hunyuan Video denoise-step measurement (same JSON contract, steps of cond+uncond forwards + CFG + Euler) -> result dict.
+    `outputs` (a dict, or None): receives what the timed steps and the timed VAE decode computed (see dump_sample)."""
     import types
     from wan2gp_b200 import _lib, ops, synth
     from wan2gp_b200.hyvideo import HYVideoDiffusionTransformer, get_rotary_pos_embed
@@ -112,6 +129,8 @@ def measure_hunyuan(workload, steps, warmup, rank, world, local_rank, dev, dist,
         barrier()
     ms = e0.elapsed_time(e1)
     launches = _lib.launch_count() - l0
+    if outputs is not None:
+        outputs["latents"] = dump_sample(latents, "latents")
     att = [(a.elapsed_time(b), w) for a, b, w in ops.TIMED.pop("attention") if w > 1e12]
     # end to end with host buffers
     n_e2e = max(1, min(args.steps, 3))
@@ -185,6 +204,8 @@ def measure_hunyuan(workload, steps, warmup, rank, world, local_rank, dev, dist,
             v1.record()
             barrier()
             vlaunch = _lib.launch_count() - l0
+            if outputs is not None:
+                outputs["vae_decode_frames"] = dump_sample(fr, "vae_decode_frames")
             del fr
             # end to end: latent on host -> uint8 frames on host
             w0, w1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
@@ -440,8 +461,9 @@ def parity_probe_wan(model, latents, tval, freqs, y_dev, dev):
 
 
 def measure_wan(workload, steps, warmup, rank, world, local_rank, dev, dist, cfg_split=False, with_vae=True, with_parity=True,
-                e2e_steps=3, with_encode=True):
-    """One Wan bench measurement -> result dict (the JSON line of the main workload, or a sub-run block)."""
+                e2e_steps=3, with_encode=True, outputs=None):
+    """One Wan bench measurement -> result dict (the JSON line of the main workload, or a sub-run block).
+    `outputs` (a dict, or None): receives what the timed steps and the timed VAE decode / encode computed (see dump_sample)."""
     from wan2gp_b200 import _lib, ops, synth
     from wan2gp_b200.pipeline import WanDenoiser
     from wan2gp_b200.wan import WanModel, WanVAE, get_rotary_pos_embed
@@ -513,6 +535,8 @@ def measure_wan(workload, steps, warmup, rank, world, local_rank, dev, dist, cfg
     if prof_range:
         torch.cuda.profiler.stop()
     ms = ev0.elapsed_time(ev1)
+    if outputs is not None:
+        outputs["latents"] = dump_sample(latents, "latents")
     launches = _lib.launch_count() + den.graph_launches - launches0      # kernels inside replayed whole-step graphs included
     att = ops.TIMED.pop("attention")
     att_ms = [a.elapsed_time(b) for a, b, _ in att]
@@ -596,6 +620,8 @@ def measure_wan(workload, steps, warmup, rank, world, local_rank, dev, dist, cfg
         if dist is not None:
             dist.all_reduce(vms, op=dist.ReduceOp.MAX)
         vms = float(vms[0]) / reps
+        if outputs is not None:
+            outputs["vae_decode_frames"] = dump_sample(fr, "vae_decode_frames")
         # end to end: latent on host -> uint8 frames on host
         zh = z.cpu().pin_memory()
         tt0 = time.time()
@@ -626,6 +652,8 @@ def measure_wan(workload, steps, warmup, rank, world, local_rank, dev, dist, cfg
                 mu = vae.encode([vid], tile_size=0)[0]
                 q1.record()
                 barrier()
+                if outputs is not None:
+                    outputs["vae_encode_latents"] = dump_sample(mu, "vae_encode_latents")
                 ems = torch.tensor([q0.elapsed_time(q1)], device=dev, dtype=torch.float64)
                 if dist is not None:
                     dist.all_reduce(ems, op=dist.ReduceOp.MAX)
@@ -672,6 +700,14 @@ def measure_wan(workload, steps, warmup, rank, world, local_rank, dev, dist, cfg
     return result, cfg, thw
 
 
+def write_outputs(out_dir, outputs):
+    if not out_dir:
+        return
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in outputs.items():
+        np.save(os.path.join(out_dir, name + ".npy"), t.numpy())
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
@@ -683,7 +719,13 @@ def main():
     ap.add_argument("--cfg-split", action="store_true", help="split each CFG pair over 2 GPUs (one 19 MB exchange per step)")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-subruns", action="store_true", help="skip the short configs[2] / configs[3] sub-runs appended at N >= 2 / N = 4")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the run, write what rank 0's timed steps (and timed VAE decode / encode) "
+                    "computed as DIR/<name>.npy, float32; outputs over 5 M elements as a fixed sample of 5 M")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs needs --impl b200")
 
     from wan2gp_b200 import synth
     cfg_name, thw, two_experts, desc = WORKLOADS[args.workload]
@@ -698,9 +740,11 @@ def main():
         if world > 1:
             import torch.distributed as dist
             dist.init_process_group("nccl", device_id=dev)
+        outputs = {} if args.dump_outputs and rank == 0 else None
         res = measure_hunyuan(args.workload, args.steps, args.warmup, rank, world, local_rank, dev, dist, with_vae=not args.no_vae and not args.cfg_split,
-                              cfg_split=args.cfg_split)
+                              cfg_split=args.cfg_split, outputs=outputs)
         if rank == 0:
+            write_outputs(args.dump_outputs, outputs)
             print(json.dumps(res))
         if dist is not None:
             dist.destroy_process_group()
@@ -730,9 +774,12 @@ def main():
     if world > 1:
         import torch.distributed as dist
         dist.init_process_group("nccl", device_id=dev)
+    outputs = {} if args.dump_outputs and rank == 0 else None
 
     result, cfg, thw = measure_wan(args.workload, args.steps, args.warmup, rank, world, local_rank, dev, dist, cfg_split=args.cfg_split,
-                                   with_vae=not args.no_vae)
+                                   with_vae=not args.no_vae, outputs=outputs)
+    if rank == 0:
+        write_outputs(args.dump_outputs, outputs)
 
     # ---- BASELINE configs[2] / configs[3] in front of the driver: short sub-runs appended to the same JSON line
     if world >= 2 and world % 2 == 0 and not args.no_subruns and not args.cfg_split and args.workload == "wan22_t2v_14b_720p81":

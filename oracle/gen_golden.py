@@ -338,6 +338,73 @@ def run_unipc(name):
     print(f"dpm++: {steps} steps, final absmean {np.abs(traj[-1]).mean():.6f}")
 
 
+def run_schedulers(name):
+    """Every reference scheduler run that tests/test_unipc_cpu.py compares with, on that module's cases and seeded inputs:
+    FlowUniPCMultistepScheduler and FlowDPMSolverMultistepScheduler (timesteps, sigmas, whole trajectories), LCMScheduler,
+    FlowMatchScheduler, Wan's EulerScheduler and Hunyuan's FlowMatchDiscreteScheduler (timesteps and final samples)."""
+    import importlib.util
+    from oracle.refshim import REFERENCE_ROOT, load_reference_unipc
+    from tests.test_unipc_cpu import CASES, inputs
+    R = load_reference_unipc()
+    out = {}
+    for steps, shift in CASES:
+        key = f"{steps}_{shift:g}"
+        ref = R.FlowUniPCMultistepScheduler(num_train_timesteps=1000, shift=1, use_dynamic_shifting=False)
+        ref.set_timesteps(steps, device="cpu", shift=shift)                      # any2video.py:519-520
+        x, vs = inputs(steps)
+        traj = []
+        for i, t in enumerate(ref.timesteps):
+            x = ref.step(vs[i], t, x, return_dict=False)[0]
+            traj.append(x.numpy().copy())
+        out.update({f"unipc_{key}_timesteps": ref.timesteps.numpy(), f"unipc_{key}_sigmas": ref.sigmas.numpy(), f"unipc_{key}_traj": np.stack(traj)})
+        ref = R.FlowDPMSolverMultistepScheduler(num_train_timesteps=1000, shift=1, use_dynamic_shifting=False)
+        ts, _ = R.retrieve_timesteps(ref, device="cpu", sigmas=R.get_sampling_sigmas(steps, shift))
+        x, vs = inputs(steps)
+        traj = []
+        for i, t in enumerate(ts):
+            x = ref.step(vs[i], t, x, return_dict=False)[0]
+            traj.append(x.numpy().copy())
+        out.update({f"dpmpp_{key}_timesteps": ts.numpy(), f"dpmpp_{key}_traj": np.stack(traj)})
+    for steps, shift in ((4, 5.0), (8, 3.0), (12, 7.0)):
+        ref = R.LCMScheduler(num_train_timesteps=1000, num_inference_steps=min(steps, 8), shift=shift)
+        ref.set_timesteps(min(steps, 8), device="cpu", shift=shift)
+        x, vs = inputs(len(ref.timesteps))
+        x = x.float()
+        for i, t in enumerate(ref.timesteps):
+            x = ref.step(vs[i].float(), t, x).prev_sample
+        out.update({f"lcm_{steps}_{shift:g}_timesteps": ref.timesteps.numpy(), f"lcm_{steps}_{shift:g}_out": x.numpy()})
+    for steps in (4, 9):
+        ref = R.FlowMatchScheduler(num_inference_steps=steps, shift=5.0, sigma_min=0, extra_one_step=True)
+        ref.timesteps = torch.tensor([1000, 934, 862, 756, 603, 410, 250, 140, 74])[:steps]
+        ref.sigmas = torch.cat([ref.timesteps / 1000, torch.tensor([0.])])
+        x, vs = inputs(steps)
+        x = x.float()
+        for i, t in enumerate(ref.timesteps):
+            x = ref.step(vs[i].float(), t, x)[0]
+        out[f"causvid_{steps}_out"] = x.numpy()
+    # Wan EulerScheduler (shared/utils/euler_scheduler.py: no third-party imports, loaded straight from the reference tree)
+    spec = importlib.util.spec_from_file_location("_ref_euler", os.path.join(REFERENCE_ROOT, "shared/utils/euler_scheduler.py"))
+    em = importlib.util.module_from_spec(spec)
+    spec.loader.exec_module(em)
+    for steps, shift in ((50, 12.0), (20, 5.0), (1, 3.0)):
+        ref = em.EulerScheduler(num_train_timesteps=1000, use_timestep_transform=True)
+        rts = ref.set_timesteps(steps, device=None, shift=shift)
+        x, vs = inputs(steps)
+        for i, t in enumerate(rts):
+            x = ref.step(vs[i], t, x, return_dict=False)[0]
+        out.update({f"euler_{steps}_{shift:g}_timesteps": rts.numpy(), f"euler_{steps}_{shift:g}_out": x.numpy()})
+    for steps, shift in ((30, 7.0), (50, 9.0), (4, 6.0)):
+        ref = R.FlowMatchDiscreteScheduler(shift=shift, reverse=True, solver="euler")
+        ref.set_timesteps(steps, device="cpu")
+        x, vs = inputs(steps)
+        x = x.float()
+        for i, t in enumerate(ref.timesteps):
+            x = ref.step(vs[i].float(), t, x, return_dict=False)[0]
+        out.update({f"flow_match_{steps}_{shift:g}_timesteps": ref.timesteps.numpy(), f"flow_match_{steps}_{shift:g}_out": x.numpy()})
+    np.savez_compressed(os.path.join(GOLDEN, f"{name}.npz"), **out)
+    print(f"{name}: {len(out)} arrays, {sum(v.nbytes for v in out.values())} bytes")
+
+
 def run_t5(name):
     """Reference T5Encoder (umT5 layout: per-layer relative position embedding) on seeded ids with a padded tail, fp32, eval mode."""
     from oracle.refshim import load_reference_t5
@@ -391,6 +458,28 @@ def run_byt5(name):
                         length=length, n_valid=n_valid, seed=0, transformers_version=transformers.__version__)
 
 
+def run_t5_cases(name):
+    """Two more reference T5Encoder calls for tests/test_t5_cpu.py: the umT5 layout (t5_small weights, seed 0) on the first 17 ids of
+    the t5_small fixture input without a mask, and the shared-position layout (byt5_tiny, seed 3) on 33 ids of which 20 are valid."""
+    from oracle.refshim import load_reference_t5
+    R = load_reference_t5()
+    out = {}
+    for cfg_name, shared_pos, seed in (("t5_small", False, 0), ("byt5_tiny", True, 3)):
+        cfg = synth.T5_CONFIGS[cfg_name]
+        enc = R.T5Encoder(cfg["vocab_size"], cfg["dim"], cfg["dim_attn"], cfg["dim_ffn"], cfg["num_heads"], cfg["num_layers"], cfg["num_buckets"],
+                          shared_pos=shared_pos).eval().float()
+        enc.load_state_dict(synth.make_t5_state_dict(cfg, seed))
+        with torch.no_grad():
+            if shared_pos:
+                ids, mask = synth.make_t5_inputs(cfg, 33, 20, seed)
+                out[f"{cfg_name}_seed{seed}"] = enc(ids[None], mask[None])[0].numpy()
+            else:
+                ids, _ = synth.make_t5_inputs(cfg, 40, 29, seed)
+                out[f"{cfg_name}_prefix17"] = enc(ids[None, :17])[0].numpy()
+    np.savez_compressed(os.path.join(GOLDEN, f"{name}.npz"), **out)
+    print(f"{name}: " + ", ".join(f"{k} {v.shape}" for k, v in out.items()))
+
+
 def run_llm(name):
     """transformers' own language-model classes on seeded synthetic weights, called the way the reference's TextEncoder.encode calls its
     model (input_ids + right-padded attention_mask, output_hidden_states=True; text_encoder_1_5.py:470-476): `Qwen2_5_VLTextModel` (the
@@ -428,4 +517,4 @@ if __name__ == "__main__":
     os.makedirs(GOLDEN, exist_ok=True)
     names = sys.argv[1:] or ["tiny", "tiny_i2v", "small", "vae_tiny", "vae_small"]
     for n in names:
-        (run_llm if n in ("qwen_tiny", "llama_tiny") else run_byt5 if n.startswith("byt5_") else run_t5 if n.startswith("t5_") else run_wan if n in WAN_CASES else run_hy if n in HY_CASES else run_hyvae if n in HYVAE_CASES else run_hyvae10 if n in HYVAE10_CASES else run_vae_enc if n in VAE_ENC_CASES else run_unipc if n == "unipc" else run_vae_tiled if n in TILED_CASES else run_hyvae_enc if n in HYVAE_ENC_CASES else run_hyvae10_enc if n in HYVAE10_ENC_CASES else run_hy_tiled if n in HY_TILED_CASES else run_vae)(n)
+        (run_schedulers if n == "schedulers" else run_t5_cases if n == "t5_cases" else run_llm if n in ("qwen_tiny", "llama_tiny") else run_byt5 if n.startswith("byt5_") else run_t5 if n.startswith("t5_") else run_wan if n in WAN_CASES else run_hy if n in HY_CASES else run_hyvae if n in HYVAE_CASES else run_hyvae10 if n in HYVAE10_CASES else run_vae_enc if n in VAE_ENC_CASES else run_unipc if n == "unipc" else run_vae_tiled if n in TILED_CASES else run_hyvae_enc if n in HYVAE_ENC_CASES else run_hyvae10_enc if n in HYVAE10_ENC_CASES else run_hy_tiled if n in HY_TILED_CASES else run_vae)(n)

@@ -1,6 +1,6 @@
 """CPU: the UniPC sampling-loop glue (SURVEY.md 8f.1) -- host coefficients of wan2gp_b200.pipeline.UniPCSchedule + the linear update
-the fused kernel applies -- against the UNMODIFIED reference FlowUniPCMultistepScheduler run in this container through
-oracle/refshim.py, and against the committed fixture (the reference does not exist on the GPU box)."""
+the fused kernel applies -- against the UNMODIFIED reference schedulers, whose runs on this module's cases and inputs are recorded in
+tests/golden/schedulers.npz, unipc.npz and dpmpp.npz (oracle/gen_golden.py)."""
 import os
 
 import numpy as np
@@ -26,6 +26,12 @@ def run_ours(steps, shift, x, vs, cls=UniPCSchedule):
     return sch, traj
 
 
+def reference_run(prefix):
+    """The reference scheduler's arrays stored under `<prefix>_*` in tests/golden/schedulers.npz."""
+    g = np.load(os.path.join(GOLDEN, "schedulers.npz"))
+    return {k[len(prefix) + 1:]: g[k] for k in g.files if k.startswith(prefix + "_")}
+
+
 def inputs(steps, seed=0):
     g = torch.Generator().manual_seed(seed)
     return torch.randn(1, 4, 2, 3, 5, generator=g, dtype=torch.float64), [torch.randn(1, 4, 2, 3, 5, generator=g, dtype=torch.float64) for _ in range(steps)]
@@ -33,18 +39,13 @@ def inputs(steps, seed=0):
 
 @pytest.mark.parametrize("steps,shift", CASES)
 def test_unipc_matches_reference_scheduler(steps, shift):
-    if not os.path.isdir("/root/reference"):
-        pytest.skip("the reference tree is only present in the build container; the committed fixture covers this elsewhere")
-    from oracle.refshim import load_reference_unipc
-    ref = load_reference_unipc().FlowUniPCMultistepScheduler(num_train_timesteps=1000, shift=1, use_dynamic_shifting=False)
-    ref.set_timesteps(steps, device="cpu", shift=shift)                      # any2video.py:519-520
+    """Timesteps, sigmas and trajectory of the reference FlowUniPCMultistepScheduler (set_timesteps as any2video.py:519-520)."""
+    ref = reference_run(f"unipc_{steps}_{shift:g}")
     x, vs = inputs(steps)
     sch, traj = run_ours(steps, shift, x, vs)
-    assert sch.timesteps == [int(t) for t in ref.timesteps]
-    assert np.allclose(sch.sigmas, ref.sigmas.numpy().astype(np.float64), rtol=0, atol=0)
-    xr = x.clone()
-    for i, t in enumerate(ref.timesteps):
-        xr = ref.step(vs[i], t, xr, return_dict=False)[0]
+    assert sch.timesteps == [int(t) for t in ref["timesteps"]]
+    assert np.allclose(sch.sigmas, ref["sigmas"].astype(np.float64), rtol=0, atol=0)
+    for i, xr in enumerate(torch.from_numpy(ref["traj"])):
         # the reference keeps its scalars in fp32; ours are fp64
         assert rel_l2(traj[i], xr) < 2e-5, (i, rel_l2(traj[i], xr))
 
@@ -73,18 +74,11 @@ def test_unipc_orders():
 @pytest.mark.parametrize("steps,shift", CASES)
 def test_dpmpp_matches_reference_scheduler(steps, shift):
     """sample_solver="dpm++" (any2video.py:523-532): host coefficients + the same fused update vs FlowDPMSolverMultistepScheduler."""
-    if not os.path.isdir("/root/reference"):
-        pytest.skip("the reference tree is only present in the build container; the committed fixture covers this elsewhere")
-    from oracle.refshim import load_reference_unipc
-    R = load_reference_unipc()
-    ref = R.FlowDPMSolverMultistepScheduler(num_train_timesteps=1000, shift=1, use_dynamic_shifting=False)
-    ts, _ = R.retrieve_timesteps(ref, device="cpu", sigmas=R.get_sampling_sigmas(steps, shift))
+    ref = reference_run(f"dpmpp_{steps}_{shift:g}")
     x, vs = inputs(steps)
     sch, traj = run_ours(steps, shift, x, vs, DPMppSchedule)
-    assert sch.timesteps == [int(t) for t in ts]
-    xr = x.clone()
-    for i, t in enumerate(ts):
-        xr = ref.step(vs[i], t, xr, return_dict=False)[0]
+    assert sch.timesteps == [int(t) for t in ref["timesteps"]]
+    for i, xr in enumerate(torch.from_numpy(ref["traj"])):
         assert rel_l2(traj[i], xr) < 2e-5, (i, rel_l2(traj[i], xr))
 
 
@@ -101,48 +95,25 @@ def test_dpmpp_matches_fixture():
 def test_single_step_solver_tables_match_reference():
     """euler / lcm / causvid are the same Euler kernel with different sigma tables: tables and whole trajectories vs the reference
     EulerScheduler-free restatement, LCMScheduler and FlowMatchScheduler (any2video.py:506-517, 533-543)."""
-    if not os.path.isdir("/root/reference"):
-        pytest.skip("the reference tree is only present in the build container")
-    from oracle.refshim import load_reference_unipc
-    R = load_reference_unipc()
+    def ours(ts, steps):
+        x, vs = inputs(steps)
+        for i in range(steps):
+            x = wan_oracle.euler_step(x, vs[i], ts[i] / 1000.0, ts[i + 1] / 1000.0)
+        return x
     for steps, shift in ((4, 5.0), (8, 3.0), (12, 7.0)):
-        ref = R.LCMScheduler(num_train_timesteps=1000, num_inference_steps=min(steps, 8), shift=shift)
-        ref.set_timesteps(min(steps, 8), device="cpu", shift=shift)
+        ref = reference_run(f"lcm_{steps}_{shift:g}")
         ts = lcm_timesteps(steps, shift)
-        assert len(ts) == min(steps, 8) + 1 and np.allclose(ts[:-1], ref.timesteps.numpy(), rtol=1e-6)
-        x, vs = inputs(len(ts) - 1)
-        xr, xo = x.clone().float(), x.clone()
-        for i, t in enumerate(ref.timesteps):
-            xr = ref.step(vs[i].float(), t, xr).prev_sample
-            xo = wan_oracle.euler_step(xo, vs[i], ts[i] / 1000.0, ts[i + 1] / 1000.0)
-        assert rel_l2(xo, xr.double()) < 1e-5
+        assert len(ts) == min(steps, 8) + 1 and np.allclose(ts[:-1], ref["timesteps"], rtol=1e-6)
+        assert rel_l2(ours(ts, len(ts) - 1), torch.from_numpy(ref["out"]).double()) < 1e-5
     for steps in (4, 9):
-        ref = R.FlowMatchScheduler(num_inference_steps=steps, shift=5.0, sigma_min=0, extra_one_step=True)
-        ref.timesteps = torch.tensor([1000, 934, 862, 756, 603, 410, 250, 140, 74])[:steps]
-        ref.sigmas = torch.cat([ref.timesteps / 1000, torch.tensor([0.])])
-        ts = causvid_timesteps(steps)
-        x, vs = inputs(steps)
-        xr, xo = x.clone().float(), x.clone()
-        for i, t in enumerate(ref.timesteps):
-            xr = ref.step(vs[i].float(), t, xr)[0]
-            xo = wan_oracle.euler_step(xo, vs[i], ts[i] / 1000.0, ts[i + 1] / 1000.0)
-        assert rel_l2(xo, xr.double()) < 1e-5
-    # Wan EulerScheduler (shared/utils/euler_scheduler.py: no third-party imports, loaded straight from the reference tree)
-    import importlib.util
-    spec = importlib.util.spec_from_file_location("_ref_euler", "/root/reference/shared/utils/euler_scheduler.py")
-    em = importlib.util.module_from_spec(spec)
-    spec.loader.exec_module(em)
+        ref = reference_run(f"causvid_{steps}")
+        assert rel_l2(ours(causvid_timesteps(steps), steps), torch.from_numpy(ref["out"]).double()) < 1e-5
+    # Wan EulerScheduler (shared/utils/euler_scheduler.py)
     for steps, shift in ((50, 12.0), (20, 5.0), (1, 3.0)):
-        ref = em.EulerScheduler(num_train_timesteps=1000, use_timestep_transform=True)
-        rts = ref.set_timesteps(steps, device=None, shift=shift)
+        ref = reference_run(f"euler_{steps}_{shift:g}")
         ts = euler_timesteps(steps, shift)
-        assert len(ts) == steps + 1 and ts[-1] == 0.0 and np.allclose(ts[:-1], rts.numpy(), rtol=1e-6)
-        x, vs = inputs(steps)
-        xr, xo = x.clone(), x.clone()
-        for i, t in enumerate(rts):
-            xr = ref.step(vs[i], t, xr, return_dict=False)[0]
-            xo = wan_oracle.euler_step(xo, vs[i], ts[i] / 1000.0, ts[i + 1] / 1000.0)
-        assert rel_l2(xo, xr) < 1e-6
+        assert len(ts) == steps + 1 and ts[-1] == 0.0 and np.allclose(ts[:-1], ref["timesteps"], rtol=1e-6)
+        assert rel_l2(ours(ts, steps), torch.from_numpy(ref["out"])) < 1e-6
 
 
 def test_denoiser_solver_selection():
@@ -155,18 +126,11 @@ def test_denoiser_solver_selection():
 
 def test_hunyuan_flow_match_table_matches_reference():
     """HunyuanDenoiser's sigma grid == FlowMatchDiscreteScheduler(shift, reverse=True, solver="euler") and its step is the Euler update."""
-    if not os.path.isdir("/root/reference"):
-        pytest.skip("the reference tree is only present in the build container")
-    from oracle.refshim import load_reference_unipc
-    R = load_reference_unipc()
     for steps, shift in ((30, 7.0), (50, 9.0), (4, 6.0)):
-        ref = R.FlowMatchDiscreteScheduler(shift=shift, reverse=True, solver="euler")
-        ref.set_timesteps(steps, device="cpu")
+        ref = reference_run(f"flow_match_{steps}_{shift:g}")
         ts = flow_match_timesteps(steps, shift)
-        assert len(ts) == steps + 1 and ts[-1] == 0.0 and np.allclose(ts[:-1], ref.timesteps.numpy(), rtol=1e-6)
-        x, vs = inputs(steps)
-        xr, xo = x.clone().float(), x.clone()
-        for i, t in enumerate(ref.timesteps):
-            xr = ref.step(vs[i].float(), t, xr, return_dict=False)[0]
+        assert len(ts) == steps + 1 and ts[-1] == 0.0 and np.allclose(ts[:-1], ref["timesteps"], rtol=1e-6)
+        xo, vs = inputs(steps)
+        for i in range(steps):
             xo = wan_oracle.euler_step(xo, vs[i], ts[i] / 1000.0, ts[i + 1] / 1000.0)
-        assert rel_l2(xo, xr.double()) < 1e-5
+        assert rel_l2(xo, torch.from_numpy(ref["out"]).double()) < 1e-5
